@@ -7,6 +7,7 @@ train_patch2pix.py:97-118), on N B200s of one node.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference algorithm (CPU oracle port) on host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's matches / scores / anchors as .npy
 
 One "step" = one image pair per GPU through the whole hot path (weak scaling: pair p of step s
 goes to rank p % N; no data-path collective, NCCL only broadcasts the pair indices and gathers
@@ -28,6 +29,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the benchmark leaves the source tree as it found it (it may be read-only)
 
 H_DEF, W_DEF, PTMAX_DEF, PANC_DEF = 480, 640, 400, 8
 MAC_CONV1, MAC_CONV2 = 152764416, 150994944        # per patch, dense count (SURVEY.md s8d)
@@ -69,7 +71,14 @@ def parse():
     ap.add_argument('--depth', type=int, default=3, help='pairs in flight per GPU (coarse stages enqueued ahead of the host sync)')
     ap.add_argument('--legacy-workload', action='store_true', help="round-1 generator (13-17 mutual matches per pair)")
     ap.add_argument('--cpu-sample-patches', type=int, default=200)
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the hot path returned in the last timed step as DIR/<name>.npy '
+                         '(fine_matches, fine_scores float32; anchors float64); with more than one GPU, each rank writes '
+                         'its own pair with a _rank<r> suffix')
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the CUDA path (--impl ours)')
+    return args
 
 
 def model_config(device, panc):
@@ -261,6 +270,26 @@ def make_workload(args):
     return make_seeded_state_dict(0, nc_init='consensus'), synthetic_pair_shifted
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res, anchors, rank=None):
+    """Write one pair's hot-path outputs (`res` [patches, 5] = fine matches x1 y1 x2 y2 + confidence, `anchors` [patches, 4]
+    int64) as .npy files, so that two builds can be compared output for output.  Past DUMP_MAX_BYTES a fixed seeded sample
+    of the rows is written, with their indices in rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {'fine_matches': res[:, :4].float(), 'fine_scores': res[:, 4].float(), 'anchors': anchors.double()}
+    n = res.shape[0]
+    cap = DUMP_MAX_BYTES // (4 * 4 + 4 + 4 * 8 + 8)
+    if n > cap:
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:cap].sort().values
+        out = {k: v[rows.to(v.device)] for k, v in out.items()}
+        out['rows'] = rows.double()
+    sfx = '' if rank is None else f'_rank{rank}'
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + sfx + '.npy'), t.cpu().numpy())
+
+
 def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
@@ -360,6 +389,7 @@ def run_ours(args):
     pinned = [(a.pin_memory(), b.pin_memory()) for a, b in imgs]
     n_patches = args.ptmax * PANC_DEF
     results = torch.zeros(max(K, 1), n_patches, 5, device=dev)
+    last_anchors = torch.zeros(n_patches, 4, dtype=torch.int64, device=dev) if args.dump_outputs else None
 
     # Two pairs are kept in flight: the coarse stage of pair i is enqueued before the host waits for the
     # mutual-match count of pair i-1 (filter_coarse's host sync), so the GPU never idles on that sync.
@@ -378,6 +408,8 @@ def run_ours(args):
         if out_slot is not None:
             results[out_slot, :, :4] = fine[0]
             results[out_slot, :, 4] = fine_p[0]
+            if last_anchors is not None and out_slot == min(K, n_mine) - 1:
+                last_anchors.copy_(cm[0])                  # the last timed step's anchors, for --dump-outputs
             if stamp:
                 step_events[out_slot].record()
                 host_stamps[out_slot] = time.perf_counter()
@@ -474,6 +506,8 @@ def run_ours(args):
         launches = net._handle.launch_count() - l0
         clocks = sampler.finish() if sampler else None
         nst = min(K, n_mine)
+        if args.dump_outputs and nst > 0:
+            dump_outputs(args.dump_outputs, results[nst - 1], last_anchors, rank if world > 1 else None)
         step_raw = [step_events[j].elapsed_time(step_events[j + 1]) for j in range(nst - 1)]
         step_ms = sorted(step_raw)
         worst = max(range(len(step_raw)), key=lambda j: step_raw[j]) if step_raw else None

@@ -1,8 +1,10 @@
-"""Generate golden vectors by running the LIVE reference (/root/reference) on CPU.
+"""Generate golden vectors by running the LIVE reference (a checkout of
+https://github.com/GrumpyZhou/patch2pix) on CPU:
 
-Run in the authoring container only (the reference does not travel to the GPU
-box):   python tests/golden/make_golden.py
-Writes tests/golden/*.npz.  The reference is imported unmodified except for the
+    PATCH2PIX_REFERENCE=/path/to/patch2pix python tests/golden/make_golden.py
+
+Writes tests/golden/*.npz; the tests only read those files, never the reference.
+The reference is imported unmodified except for the
 two import-time shims documented in SURVEY.md Appendix B (skip the ResNet
 checkpoint download; do not .cuda() the NC net on a CPU-only host).
 """
@@ -17,7 +19,9 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, '/root/reference')
+if not os.environ.get('PATCH2PIX_REFERENCE'):
+    sys.exit('set PATCH2PIX_REFERENCE to a checkout of the reference patch2pix repository')
+sys.path.insert(0, os.environ['PATCH2PIX_REFERENCE'])
 warnings.filterwarnings('ignore')
 
 import networks.resnet as resnet                                   # noqa: E402

@@ -129,6 +129,29 @@ def test_bench_reference_arm_line():
     assert line['e2e']['h2d_bytes_per_step'] == 0 and line['unit'] == 'pairs/s'
 
 
+def test_bench_dump_outputs_files(tmp_path):
+    """bench.py --dump-outputs: one .npy per returned array, float32 / float64, values as given; a fixed seeded row sample
+    past the size cap."""
+    import numpy as np
+    code = ('import sys, torch; import bench; d = sys.argv[1]; g = torch.Generator().manual_seed(0); '
+            'res = torch.randn(300, 5, generator=g); anc = torch.randint(-8, 640, (300, 4), generator=g); '
+            'bench.dump_outputs(d + "/all", res, anc); bench.DUMP_MAX_BYTES = 60 * 50; '
+            'bench.dump_outputs(d + "/cut", res, anc, rank=1); bench.dump_outputs(d + "/cut2", res, anc, rank=1); '
+            'torch.save((res, anc), d + "/in.pt")')
+    r = subprocess.run([sys.executable, '-c', code, str(tmp_path)], capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    res, anc = torch.load(tmp_path / 'in.pt')
+    full = {f.name: np.load(f) for f in (tmp_path / 'all').iterdir()}
+    assert sorted(full) == ['anchors.npy', 'fine_matches.npy', 'fine_scores.npy']
+    assert full['fine_matches.npy'].dtype == np.float32 and np.array_equal(full['fine_matches.npy'], res[:, :4].numpy())
+    assert full['fine_scores.npy'].dtype == np.float32 and np.array_equal(full['fine_scores.npy'], res[:, 4].numpy())
+    assert full['anchors.npy'].dtype == np.float64 and np.array_equal(full['anchors.npy'], anc.numpy())
+    rows = np.load(tmp_path / 'cut' / 'rows_rank1.npy').astype(np.int64)
+    assert len(rows) == 50 and np.array_equal(rows, np.load(tmp_path / 'cut2' / 'rows_rank1.npy'))
+    assert np.array_equal(np.load(tmp_path / 'cut' / 'fine_matches_rank1.npy'), res[rows, :4].numpy())
+    assert np.array_equal(np.load(tmp_path / 'cut' / 'anchors_rank1.npy'), anc[rows].numpy())
+
+
 def test_load_checkpoint_parses_the_released_file_format(tmp_path, seeded_sd):
     """utils/eval/model_helper.py:28-62: released checkpoints are pickled dicts holding a Namespace; the loader
     must read them (weights_only=False), reject other architectures, and -- with no GPU here -- stop at the
